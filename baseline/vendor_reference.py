@@ -3,8 +3,8 @@
 The reference is a script tree without setup.py / pyproject.toml, so `pip install --target baseline/_ref /root/reference`
 has nothing to install (DESIGN.md section 2); the equivalent for a script tree is a verbatim copy of its importable
 modules. `baseline/_ref/` is git-ignored (never part of this repository's history) but not gpurun-ignored. The copy is
-byte-identical: `bench.py --impl reference` / `--impl reference-cuda` and tests/test_gpu_vs_reference.py import it from there
-under its own module names (`training`, `torch_utils`, `dnnlib`), never mixed into the product path.
+byte-identical: `bench.py --impl reference` / `--impl reference-cuda` and oracle/make_golden_vs_reference.py import it from
+there under its own module names (`training`, `torch_utils`, `dnnlib`), never mixed into the product path.
 
     python baseline/vendor_reference.py            # no-op when /root/reference is absent (GPU box: uses the shipped copy)
 """

@@ -7,6 +7,7 @@ neural-rendering resolution, 48+48 samples per ray).
     python bench.py --impl reference ...          # the UNMODIFIED reference (baseline/_ref) on the host cores, same config
     python bench.py --impl reference-cuda ...     # the UNMODIFIED reference on the GPU through its own JIT-built plugins
     python bench.py --workload {seg2cat_smoke,seg2cat_512,seg2face_512,edge2car_128}     # BASELINE.json configs 1-4
+    python bench.py ... --dump-outputs DIR        # also write the outputs of the last timed step as DIR/<name>.npy
 
 A step is one `G.synthesis(ws, c, noise_mode='const', neural_rendering_resolution=128)` of
 TriPlaneSemanticEntangleGenerator on a batch of 4 (BASELINE configs[1]); weights are seeded random, inputs synthetic.
@@ -258,8 +259,8 @@ def run_train_step_arm(args):
         cfg['mbstd_group'] = min(cfg['mbstd_group'], args.batch)
     st = ts.build(cfg, dev, rank=rank, num_gpus=world, seed=0)
     batch = ts.synthetic_batch(cfg, dev, 100 + rank)
-    steps = args.steps if args.steps != 20 else 16                 # default: one full lazy-regularisation period
-    warm = max(args.warmup if args.warmup != 5 else 3, 3)
+    steps = args.steps
+    warm = max(args.warmup, 3)
 
     def barrier():
         if world > 1:
@@ -350,13 +351,33 @@ def render_traffic(workload, B):
     return None, None
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, outputs, limit=DUMP_LIMIT_BYTES):
+    """Write each output as out_dir/<name>.npy in float32. Above `limit` bytes in all, every output is cut to a share of
+    the limit proportional to its size: a sorted sample of its flattened elements drawn with a fixed seed, so two runs of
+    the same workload keep the same elements."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: v.numpy().astype(np.float32) for k, v in outputs.items()}
+    total = sum(a.size for a in arrays.values())
+    budget = (limit - 4096 * len(arrays)) // 4          # 4 KiB per file covers the .npy header
+    for k, a in arrays.items():
+        if total > budget:
+            keep = a.size * budget // total
+            a = a.reshape(-1)[np.sort(np.random.RandomState(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(out_dir, k + '.npy'), a)
+
+
 # ---------------------------------------------------------------------------------------------
 def main():
     global WORKLOAD
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=20)
-    ap.add_argument('--warmup', type=int, default=5)
+    ap.add_argument('--steps', type=int, default=None,
+                    help='timed steps (default: 20; 16 for train_step, one full lazy-regularisation period)')
+    ap.add_argument('--warmup', type=int, default=None, help='untimed steps before the timed ones (default: 5; 3 for train_step)')
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference', 'reference-cuda'])
     ap.add_argument('--workload', default=WORKLOAD, choices=['seg2cat_smoke', 'seg2cat_512', 'seg2face_512', 'edge2car_128', 'train_step'],
                     help='BASELINE.json configs 1-4 (default: configs[1], the metric\'s configuration)')
@@ -365,7 +386,18 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--force-fp32', action='store_true', help='run the SR stacks in fp32 (reference default is fp16)')
     ap.add_argument('--no-graph', action='store_true', help='launch every kernel from Python instead of replaying a CUDA graph')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs of the last timed step as DIR/<name>.npy (float32); when they exceed 64 MB in all, '
+                         'each is replaced by the same fixed-seed sample of its flattened elements')
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 16 if args.workload == 'train_step' else 20
+    if args.warmup is None:
+        args.warmup = 3 if args.workload == 'train_step' else 5
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.workload == 'train_step' or args.impl != 'ours'):
+        ap.error('--dump-outputs applies to the G.synthesis benchmark of this repository (--impl ours, not train_step)')
     if args.workload == 'train_step':
         if args.impl == 'reference':
             raise SystemExit('--workload train_step has the arms `ours` and `reference-cuda` (a CPU train step takes minutes per image)')
@@ -451,6 +483,8 @@ def main():
     e1.record()
     barrier()
     ms = max_over_ranks(e0.elapsed_time(e1))
+    # graph replay reuses its output tensors, so the last timed step's outputs are copied out before anything else runs
+    dumped = {k: v.detach().float().cpu() for k, v in out.items()} if args.dump_outputs and rank == 0 else None
     launches = graphed.native_launches if graphed is not None else (_lib.launch_count - launches0) / args.steps
     kev = native.kernel_events
     native.kernel_events = None
@@ -605,6 +639,8 @@ def main():
         'stock_cuda': stock_cuda, 'vs_stock_cuda': vs_stock,
     }
     print(json.dumps(line), flush=True)
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
 

@@ -1,54 +1,59 @@
-"""Live comparison with the reference's own PyTorch/CUDA path (the oracle of record, SURVEY 8c) on the GPU box.
+"""Comparison with the reference's own PyTorch/CUDA path (the oracle of record, SURVEY 8c).
 
-baseline/_ref is a byte-identical copy of the reference (baseline/vendor_reference.py; git-ignored, shipped by gpurun). Its
-modules import under their own names (`training.*`, `torch_utils.*`), the product's under `pix2pix3d_b200.*`, so both
-generators live in one process with identical seeded weights and identical injected renderer noise. The reference's CUDA
-plugins are JIT-built by its own custom_ops.get_plugin on first use (about a minute)."""
+tests/golden/vs_reference_*.npz hold what the unmodified reference computed on a B200 through its JIT-built plugins and
+cuDNN for the inputs below (oracle/make_golden_vs_reference.py): seeded generator weights, seeded ws / c, and the
+renderer's two random draws fed in from seeded tensors. Inputs are regenerated from their seeds and checked against stored
+digests; outputs are kept as a fixed sample of their elements, on which this package's results are compared."""
 import os
 import sys
+import warnings
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import ROOT, rel_err
+from conftest import ROOT, load_golden, rel_err
 
 sys.path.insert(0, os.path.join(ROOT, 'baseline'))
+import make_golden_vs_reference as M  # noqa: E402
 import ref_harness as rh  # noqa: E402
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not rh.available(), reason='baseline/_ref not vendored')]
+pytestmark = pytest.mark.gpu
 
 
-def _both(workload, batch, force_fp32, seed_in=7):
+def _ours(name):
+    """This package's G.synthesis on the golden's inputs; returns (outputs sampled as stored, golden)."""
     from pix2pix3d_b200 import configs
+    workload, batch, force_fp32 = M.SYNTH_CASES[name]
+    g = load_golden(name)
     dev = torch.device('cuda')
-    torch.backends.cudnn.allow_tf32 = False          # the reference's fp32 convolutions must be true fp32 for a 1e-3 comparison
+    torch.backends.cudnn.allow_tf32 = False
     torch.backends.cuda.matmul.allow_tf32 = False
     w = configs.WORKLOADS[workload]
-    G_ref = rh.build_generator(workload, seed=0, device=dev)
     G = configs.build_generator(workload, seed=0, device=dev, with_mapping=False)
-    sd_r, sd = G_ref.state_dict(), G.state_dict()
-    assert sd_r.keys() == sd.keys() and all(torch.equal(sd_r[k], sd[k]) for k in sd), 'arms must hold identical weights'
+    keys, sumsq = M.state_dict_digest(G)
+    assert list(keys) == list(g['sd_keys']) and np.array_equal(sumsq, g['sd_digest']), 'weights must be the reference\'s'
     rk = G.rendering_kwargs
-    nrr, Sc, Sf = w['nrr'], rk['depth_resolution'], rk['depth_resolution_importance']
-    ws = configs.synthetic_ws(batch, G.backbone.num_ws, seed_in).to(dev)
-    c = configs.camera_labels(batch, seed_in + 1, w['preset']).to(dev)
-    g = torch.Generator().manual_seed(seed_in + 2)
-    jitter = torch.rand(batch, nrr * nrr, Sc, 1, generator=g).to(dev)
-    u = torch.rand(batch * nrr * nrr, Sf, generator=g).to(dev)
+    nrr = w['nrr']
+    ws, c, jitter, u = M.synthesis_inputs(workload, batch, G.backbone.num_ws, nrr, rk['depth_resolution'],
+                                          rk['depth_resolution_importance'])
+    for k, t in (('ws', ws), ('c', c), ('jitter', jitter), ('u', u)):
+        assert M.digest(t) == g[k + '_digest'], f'input {k} must be the reference\'s'
     kw = dict(noise_mode='const', neural_rendering_resolution=nrr, force_fp32=force_fp32)
-    with torch.no_grad():
-        with rh.replay_rand(jitter, u):
-            out_ref = G_ref.synthesis(ws, c, **kw)
-        with rh.replay_rand(jitter, u):
-            out = G.synthesis(ws, c, **kw)
-    return out, out_ref
+    with torch.no_grad(), rh.replay_rand(jitter.to(dev), u.to(dev)):
+        out = G.synthesis(ws.to(dev), c.to(dev), **kw)
+    assert sorted(out) == list(g['out_keys'])
+    for k, v in out.items():
+        assert tuple(v.shape) == tuple(g['shape_' + k]), k
+    return {k: M.sampled(v.float().cpu().numpy(), M.SYNTH_SAMPLE) for k, v in out.items()}, g
 
 
 @pytest.mark.parametrize('workload,batch', [('seg2cat_512', 2), ('edge2car_128', 3)])
 def test_synthesis_matches_reference_cuda_path_fp32(workload, batch):
-    out, out_ref = _both(workload, batch, True)
-    errs = {k: rel_err(out[k].float().cpu().numpy(), out_ref[k].float().cpu().numpy()) for k in out_ref}
+    name = f'vs_reference_{workload}_fp32'
+    assert M.SYNTH_CASES[name] == (workload, batch, True)
+    out, g = _ours(name)
+    errs = {k: rel_err(v, g['out_' + k]) for k, v in out.items()}
     print('VS-REFERENCE-CUDA fp32', workload, errs)
     for k, e in errs.items():
         assert e < 1e-3, (k, errs)
@@ -56,8 +61,8 @@ def test_synthesis_matches_reference_cuda_path_fp32(workload, batch):
 
 def test_synthesis_matches_reference_cuda_path_default_dtypes():
     """SR in fp16 on both sides (superresolution.py:304): the two fp16 paths round differently, so the bound is fp16-sized."""
-    out, out_ref = _both('seg2cat_512', 2, False)
-    errs = {k: rel_err(out[k].float().cpu().numpy(), out_ref[k].float().cpu().numpy()) for k in out_ref}
+    out, g = _ours('vs_reference_seg2cat_512_default')
+    errs = {k: rel_err(v, g['out_' + k]) for k, v in out.items()}
     print('VS-REFERENCE-CUDA default dtypes', errs)
     for k in ('image_raw', 'image_depth', 'semantic_raw'):
         assert errs[k] < 1e-3, (k, errs)
@@ -66,94 +71,56 @@ def test_synthesis_matches_reference_cuda_path_default_dtypes():
 
 
 def test_reference_op_wrappers_run_on_libp3d_plugins():
-    """INTEGRATION.md section 2: the reference's own torch_utils/ops/{bias_act,upfirdn2d}.py, unmodified, with this package's
-    `custom_ops.get_plugin` objects in place of the JIT-built pybind modules -- compared with the same wrappers on the
-    reference's stock plugins (forward and first-order gradients; e.g. the stock CUDA path does not clamp the gradient of a
-    clamped `linear` activation, bias_act.py:164-167 saves no `y` for it, and neither may the replacement)."""
-    rh.import_reference()
-    import torch_utils.ops.bias_act as r_ba
-    import torch_utils.ops.upfirdn2d as r_up
+    """bias_act / upfirdn2d (forward, first- and second-order gradients) on libp3d against the reference's wrappers on its
+    stock plugins (e.g. the stock CUDA path does not clamp the gradient of a clamped `linear` activation,
+    bias_act.py:164-167 saves no `y` for it, and neither may this package). The forward also goes through the plugin
+    objects `custom_ops.get_plugin` hands to the reference's wrappers, with the arguments those wrappers pass."""
     from pix2pix3d_b200.torch_utils import custom_ops as ours
+    from pix2pix3d_b200.torch_utils.ops import bias_act as ba, upfirdn2d as up
+    g = load_golden('vs_reference_bias_act_upfirdn2d')
     dev = torch.device('cuda')
-    assert r_ba._init() and r_up._init()                       # JIT-build / load the stock plugins
-    stock = (r_ba._plugin, r_up._plugin)
-    mine = (ours.get_plugin('bias_act_plugin', sources=['bias_act.cpp', 'bias_act.cu']),
-            ours.get_plugin('upfirdn2d_plugin', sources=['upfirdn2d.cpp', 'upfirdn2d.cu']))
-    torch.manual_seed(0)
-    x = torch.randn(3, 8, 33, 31, device=dev, requires_grad=True)
-    b = torch.randn(8, device=dev, requires_grad=True)
-    f = r_up.setup_filter([1, 3, 3, 1], device=dev)
+    x, b = M.ops_inputs(dev)
+    assert M.digest(x) == g['x_digest'] and M.digest(b) == g['b_digest'], 'inputs must be the reference\'s'
+    f = torch.from_numpy(g['f']).to(dev)
+    got = M.bias_act_upfirdn2d_cases(ba.bias_act, up.upfirdn2d, x, b, f)
+    assert [n for n, _ in got] == list(g['names'])
+    want = {}
+    for i, (n, a) in enumerate(got):
+        assert a.shape == tuple(g[f'shape{i:03d}']), n
+        want[n] = g[f'res{i:03d}']
+        assert rel_err(M.sampled(a, M.OPS_SAMPLE), want[n]) < 2e-6, n
 
-    def run_all():
-        res = []
+    p_ba = ours.get_plugin('bias_act_plugin', sources=['bias_act.cpp', 'bias_act.cu'])
+    p_up = ours.get_plugin('upfirdn2d_plugin', sources=['upfirdn2d.cpp', 'upfirdn2d.cu'])
+    null = torch.empty([0], device=dev)
+    with torch.no_grad():
         for act in ('lrelu', 'swish', 'linear', 'sigmoid', 'softplus'):
-            y = r_ba.bias_act(x, b, act=act, clamp=1.5, impl='cuda')
-            gx, gb = torch.autograd.grad(y.square().sum(), [x, b], create_graph=True)
-            (ggx,) = torch.autograd.grad(gx.square().sum() + gb.square().sum(), [x], allow_unused=True)
-            res += [('bias_act ' + act, y), ('bias_act dx ' + act, gx), ('bias_act db ' + act, gb)]
-            if ggx is not None:
-                res.append(('bias_act d2 ' + act, ggx))
-        for kw in (dict(up=2, padding=[2, 1, 2, 1], gain=4), dict(down=2, padding=[1, 1, 1, 1]), dict(padding=[1, 1, 1, 1], gain=4)):
-            y = r_up.upfirdn2d(x, f, impl='cuda', **kw)
-            (gx,) = torch.autograd.grad(y.square().sum(), [x])
-            res += [(f'upfirdn2d {kw}', y), (f'upfirdn2d dx {kw}', gx)]
-        return [(n, t.detach().float().cpu().numpy()) for n, t in res]
-
-    try:
-        want = run_all()
-        r_ba._plugin, r_up._plugin = mine
-        got = run_all()
-    finally:
-        r_ba._plugin, r_up._plugin = stock
-    assert len(want) == len(got)
-    for (n, w), (_, g) in zip(want, got):
-        assert rel_err(g, w) < 2e-6, n
+            spec, alpha, gain, clamp = ba._resolve(act, None, None, 1.5)
+            y = p_ba.bias_act(x, b, null, null, null, 0, 1, spec.cuda_idx, alpha, gain, clamp)
+            assert rel_err(M.sampled(y.cpu().numpy(), M.OPS_SAMPLE), want['bias_act ' + act]) < 2e-6, act
+        for kw, (upxy, downxy, pads, gain) in (("{'up': 2, 'padding': [2, 1, 2, 1], 'gain': 4}", (2, 1, (2, 1, 2, 1), 4.0)),
+                                                ("{'down': 2, 'padding': [1, 1, 1, 1]}", (1, 2, (1, 1, 1, 1), 1.0)),
+                                                ("{'padding': [1, 1, 1, 1], 'gain': 4}", (1, 1, (1, 1, 1, 1), 4.0))):
+            y = p_up.upfirdn2d(x, f, upxy, upxy, downxy, downxy, *pads, False, gain)
+            assert rel_err(M.sampled(y.cpu().numpy(), M.OPS_SAMPLE), want['upfirdn2d ' + kw]) < 2e-6, kw
 
 
 def test_reference_filtered_lrelu_wrapper_runs_on_libp3d_plugin():
-    """The reference's torch_utils/ops/filtered_lrelu.py (autograd class, sign-tensor hand-off between forward and backward,
-    fallback on rc = -1) unmodified, once on its stock JIT-built plugin and once on this package's `filtered_lrelu_plugin`."""
-    import scipy.signal
-    rh.import_reference()
-    import torch_utils.ops.filtered_lrelu as r_fl
-    from pix2pix3d_b200.torch_utils import custom_ops as ours
+    """filtered_lrelu (forward and gradients, fp32 and fp16) on libp3d against the reference's
+    torch_utils/ops/filtered_lrelu.py on its stock JIT-built plugin."""
+    from pix2pix3d_b200.torch_utils.ops import filtered_lrelu as fl
+    g = load_golden('vs_reference_filtered_lrelu')
     dev = torch.device('cuda')
-    assert r_fl._init()
-    stock = r_fl._plugin
-    mine = ours.get_plugin('filtered_lrelu_plugin', sources=['filtered_lrelu.cpp'])
-    torch.manual_seed(0)
-    k12 = torch.as_tensor(scipy.signal.firwin(numtaps=12, cutoff=0.25, width=0.3, fs=2.0), dtype=torch.float32, device=dev)
-    f4 = torch.tensor([1., 3., 3., 1.], device=dev)
-    f4 = torch.outer(f4, f4) / 64
-    cases = [dict(fu=k12, fd=k12, up=2, down=2, padding=[10, 9, 10, 9], gain=1.4, slope=0.2, clamp=256),
-             dict(fu=f4, fd=f4, up=2, down=2, padding=[3, 2, 3, 2], gain=1.0, slope=0.2, clamp=0.8),
-             dict(fu=k12, fd=None, up=2, down=1, padding=[5, 6, 5, 6], gain=2 ** 0.5, slope=0.2, clamp=None, flip_filter=True)]
-
-    def run_all():
-        res = []
-        for kw in cases:
-            # the stock plugin has no fused kernel for 2-D filters at up = down = 2 (filtered_lrelu.cu:1252-1259 lists none):
-            # it composes upfirdn2d + act + upfirdn2d, which in fp16 rounds the up-sampled tensor and so takes other lrelu /
-            # clamp branches than a kernel that keeps fp32 inside; compare that case in fp32 only
-            for dtype in ((torch.float32, torch.float16) if kw['fu'].ndim == 1 else (torch.float32,)):
-                x = torch.randn(2, 6, 25, 20, device=dev, generator=torch.Generator(dev).manual_seed(1)).to(dtype).requires_grad_(True)
-                b = torch.randn(6, device=dev, generator=torch.Generator(dev).manual_seed(2)).to(dtype).requires_grad_(True)
-                y = r_fl.filtered_lrelu(x, b=b, impl='cuda', **kw)
-                gx, gb = torch.autograd.grad(y.float().square().sum(), [x, b])
-                res += [(dtype, y), (dtype, gx), (dtype, gb)]
-        return [(d, t.detach().float().cpu().numpy()) for d, t in res]
-
-    import warnings
-    try:
-        with warnings.catch_warnings():
-            warnings.simplefilter('ignore', RuntimeWarning)
-            want = run_all()
-            r_fl._plugin = mine
-            got = run_all()
-    finally:
-        r_fl._plugin = stock
-    for i, ((d, w), (_, g)) in enumerate(zip(want, got)):
+    x, b = M.filtered_lrelu_inputs(dev)
+    assert M.digest(x) == g['x_digest'] and M.digest(b) == g['b_digest'], 'inputs must be the reference\'s'
+    with warnings.catch_warnings():
+        warnings.simplefilter('ignore', RuntimeWarning)
+        got = M.filtered_lrelu_cases(fl.filtered_lrelu, x, b, M.filtered_lrelu_filters(dev))
+    assert [d for d, _ in got] == list(g['dtypes'])
+    for i, (d, a) in enumerate(got):
+        assert a.shape == tuple(g[f'shape{i:03d}']), i
+        a, w = M.sampled(a, M.OPS_SAMPLE), g[f'res{i:03d}']
         # fp16: both kernels hold fp32 inside but sum in different orders; an element within rounding of 0 / the clamp may
         # take the other branch, which moves single gradient entries
-        tol = 2e-5 if d == torch.float32 else 2e-2
-        assert rel_err(g, w) < tol, (i, d, rel_err(g, w))
+        tol = 2e-5 if d == str(torch.float32) else 2e-2
+        assert rel_err(a, w) < tol, (i, d, rel_err(a, w))
