@@ -379,9 +379,12 @@ __global__ void __launch_bounds__(192, 2) conv_gemm_kernel(const __grid_constant
             if (!pix_ok) continue;
             const int ch0 = n0 + c0;
             if (a.partial) {
-                // split-K: raw accumulators of this k-range; conv_splitk_finish_kernel sums the ranges and applies the epilogue
+                // split-K: raw accumulators of this k-range; conv_splitk_finish_kernel sums the ranges and applies the epilogue.
+                // Partial rows are Cout_pad wide: when Cout_pad > BN is not a multiple of BN, the last channel tile reaches past
+                // the row, and those columns would land in the next pixel's row.
+                if (ch0 >= a.Cout_pad) continue;
                 float* pp = a.partial + P.p0 + ((((size_t)ksplit * (gridDim.z / a.splits) + b) * P.gH + gy) * P.gW + gx) * a.Cout_pad + ch0;
-                const int ncols = min(32, a.BN - c0);
+                const int ncols = min(min(32, a.BN - c0), a.Cout_pad - ch0);
 #pragma unroll
                 for (int j = 0; j < 4; ++j)
                     if (8 * j < ncols) {

@@ -149,11 +149,15 @@ def test_graphed_synthesis_replays_and_matches_eager():
     assert a['image'].shape == e['image'].shape
 
 
-@pytest.mark.parametrize('workload,batch', [('seg2cat_512', 3), ('seg2face_512', 2), ('edge2car_128', 5)])
-def test_full_size_workloads_engine_matches_generic_path(workload, batch):
+@pytest.mark.parametrize('workload,batch,noise_mode', [
+    pytest.param('seg2cat_512', 3, 'const', id='seg2cat_512-3'), pytest.param('seg2face_512', 2, 'const', id='seg2face_512-2'),
+    pytest.param('edge2car_128', 5, 'const', id='edge2car_128-5'), pytest.param('seg2cat_512', 3, 'random', id='seg2cat_512-3-random')])
+def test_full_size_workloads_engine_matches_generic_path(workload, batch, noise_mode):
     """BASELINE configs 2-4 at their real channel counts and resolutions (odd batch sizes on purpose): the whole-generator
     tensor-core path against the op-by-op formulation of the same modules (ATen convolutions + libp3d bias_act/upfirdn2d,
-    staged or fused renderer), with identical renderer noise."""
+    staged or fused renderer), with identical renderer noise. noise_mode='random' (the default of G.synthesis) draws one
+    noise image per sample and layer; both paths must draw them, and then the renderer's jitter and `u`, in the same order
+    from the same seed, which the generator state after the call shows."""
     from pix2pix3d_b200 import _lib, configs, engine
     torch.backends.cudnn.allow_tf32 = False
     torch.backends.cuda.matmul.allow_tf32 = False
@@ -161,24 +165,26 @@ def test_full_size_workloads_engine_matches_generic_path(workload, batch):
     G = configs.build_generator(workload, seed=3, device='cuda', with_mapping=False)
     ws = configs.synthetic_ws(batch, G.backbone.num_ws, seed=4).cuda()
     c = configs.camera_labels(batch, seed=5, preset=w['preset']).cuda()
-    kw = dict(noise_mode='const', neural_rendering_resolution=w['nrr'])
+    kw = dict(noise_mode=noise_mode, neural_rendering_resolution=w['nrr'])
 
     def run():
-        torch.manual_seed(77)                     # same jitter / u draws for both paths
+        torch.manual_seed(77)                     # same noise / jitter / u draws for both paths
         with torch.no_grad():
-            return {k: v.float().clone() for k, v in G.synthesis(ws, c, **kw).items()}
+            out = {k: v.float().clone() for k, v in G.synthesis(ws, c, **kw).items()}
+        return out, (torch.get_rng_state(), torch.cuda.get_rng_state())
 
     n0 = _lib.launch_count
-    fast = run()
+    fast, rng_fast = run()
     n_fast = _lib.launch_count - n0
     engine.enabled = False
     try:
         n0 = _lib.launch_count
-        ref = run()
+        ref, rng_ref = run()
         n_ref = _lib.launch_count - n0
     finally:
         engine.enabled = True
     assert n_fast > 60 and n_ref > 0
+    assert all(torch.equal(a, b) for a, b in zip(rng_fast, rng_ref)), 'the two paths consumed the generators differently'
     # The two paths produce tri-planes that differ at fp32 rounding level (3-pass tensor-core split vs cuDNN); a handful of
     # rays then take a different searchsorted branch in the importance sampling, which moves single pixels by ~1e-3 of the
     # range. Bound the worst pixel loosely and the average tightly.

@@ -277,7 +277,8 @@ def test_fused_torgb_tail_matches_upsample_plus_conv(cout, hw, split, nchw):
 @pytest.mark.parametrize('split', [False, True])
 def test_cta_pair_kernel_256_channel_tiles(split):
     """Layers with >= 256 output channels and >= 74 tile pairs run on CTA pairs (cta_group::2, one 256x256 tile per two
-    SMs); the result must equal the single-CTA kernels' (P3D_CONV_PAIR=0 is read once per process, so compare with torch)."""
+    SMs), here with weights shared by the batch, against float64 torch. tcconv.launch_flags is read on every call;
+    test_gpu_kernel_instances.py runs per-sample-weight pair launches through the single-CTA kernels too and compares."""
     from pix2pix3d_b200 import tcconv
     torch.manual_seed(21)
     b, c, h, w, cout = 2, 128, 96, 80, 512           # 2 * ceil(96*80/256) * 2 = 120 tile pairs, odd tile edges
