@@ -469,6 +469,26 @@ int p3d_fir_act_nhwc_sep(const void* x, int in_dtype, const float fx[4], const f
 
 
 
+/* ---------------------------------------------------------------------------------------------
+ * Mesh extraction (applications/extract_mesh.py:84-96: mcubes.marching_cubes on the dense sigma grid)
+ * ------------------------------------------------------------------------------------------- */
+
+/* Marching cubes on a dense fp32 grid volume [nx][ny][nz] (C order), each side >= 2 (pix2pix3d_b200/csrc/marching_cubes.cu;
+ * the mesh is defined in oracle/p3d_oracle/mesh.py). A point is inside when (double)v > threshold (NaN is outside). One
+ * vertex per grid edge p -> p + e_axis whose endpoints differ in inside-ness, at p + t e_axis, t = (threshold - v_p) /
+ * (v_{p+e} - v_p) in float64, ordered by owning point p in C order and by axis within a point; faces are listed by cube in
+ * C order and in table order inside a cube, oriented outward (normals toward lower values). No atomics: the output depends
+ * only on the input.
+ * Two calls on one workspace of p3d_marching_cubes_workspace_bytes() bytes (P3D_BAD_ARG there for a side < 2 or a grid of
+ * 2^40 points or more): p3d_marching_cubes_count writes counts[2] = {V, F} (device int64); the caller allocates
+ * vertices [V,3] float64 (index coordinates) and faces [F,3] int64 and calls p3d_marching_cubes_emit with the same volume,
+ * threshold and workspace. Vertex ids are int32 in the workspace: V must be < 2^31. */
+int64_t p3d_marching_cubes_workspace_bytes(int64_t nx, int64_t ny, int64_t nz);
+int p3d_marching_cubes_count(const float* volume, int64_t nx, int64_t ny, int64_t nz, double threshold,
+                             void* workspace, int64_t workspace_bytes, int64_t* counts, p3d_stream_t stream);
+int p3d_marching_cubes_emit(const float* volume, int64_t nx, int64_t ny, int64_t nz, double threshold,
+                            void* workspace, int64_t workspace_bytes, double* vertices, int64_t* faces, p3d_stream_t stream);
+
 /* upsample2d(img, f) with up=2 (upfirdn2d.py:315-350) on an fp32 NHWC image: [B,H,W,C] -> [B,2H,2W,C]. */
 int p3d_upsample2x_nhwc(const float* x, const float* f, float* y, int B, int H, int W, int C, p3d_stream_t stream);
 

@@ -10,7 +10,7 @@ import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'libp3d.so')
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 _lib = None
 
@@ -124,6 +124,11 @@ _SIGNATURES = {
     'p3d_fir_act_nhwc_sep': (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int,
                                      c_int, c_int, c_int, c_float, c_int, c_float, c_float, c_float, c_int64, c_void_p]),
     'p3d_upsample2x_nhwc': (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
+    'p3d_marching_cubes_workspace_bytes': (c_int64, [c_int64, c_int64, c_int64]),
+    'p3d_marching_cubes_count': (c_int, [c_void_p, c_int64, c_int64, c_int64, ctypes.c_double, c_void_p, c_int64, c_void_p,
+                                         c_void_p]),
+    'p3d_marching_cubes_emit': (c_int, [c_void_p, c_int64, c_int64, c_int64, ctypes.c_double, c_void_p, c_int64, c_void_p,
+                                        c_void_p, c_void_p]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

@@ -262,11 +262,13 @@ def render_fwd(planes_nhwc, dec, ray_origins, ray_dirs, depths_coarse, u, box_wa
     return feat, depth, wsum
 
 
-def run_model(planes_nhwc, dec, coords, box_warp, impl=None, sigma_only=False):
+def run_model(planes_nhwc, dec, coords, box_warp, impl=None, sigma_only=False, out_sigma=None):
     """Fused sample_from_planes + decoder: coords [B,M,3] -> (rgb [B,M,C], sigma [B,M,1]).
 
     `impl`: 'auto' / 'tc' run the tensor-core query (p3d_run_model_tc), 'simt' the CUDA-core kernel.
-    `sigma_only` (tensor-core query): skip the colours and return (None, sigma) -- the mesh-extraction query."""
+    `sigma_only` (tensor-core query): skip the colours and return (None, sigma) -- the mesh-extraction query.
+    `out_sigma`: optional contiguous fp32 tensor of B*M elements on the planes' device that receives the densities in
+    place of a new [B,M,1] tensor (any shape, e.g. a slab of a dense grid); it is returned as `sigma`."""
     B, _, H, W, C = planes_nhwc.shape
     assert C == 32 and planes_nhwc.dtype == torch.float32
     impl = impl or render_impl
@@ -283,7 +285,13 @@ def run_model(planes_nhwc, dec, coords, box_warp, impl=None, sigma_only=False):
     dev = planes_nhwc.device
     sigma_only = bool(sigma_only) and use_tc
     rgb = None if sigma_only else torch.empty(B, M, dec.out_channels, device=dev, dtype=torch.float32)
-    sigma = torch.empty(B, M, 1, device=dev, dtype=torch.float32)
+    if out_sigma is None:
+        sigma = torch.empty(B, M, 1, device=dev, dtype=torch.float32)
+    else:
+        if not (out_sigma.device == dev and out_sigma.dtype == torch.float32 and out_sigma.is_contiguous()
+                and out_sigma.numel() == B * M):
+            raise ValueError(f'out_sigma must be a contiguous float32 tensor of {B * M} elements on {dev}')
+        sigma = out_sigma
     masks = (ctypes.c_uint32 * 2)(dec.masks[0], dec.masks[1])
     with torch.cuda.device(dev):
         if use_tc:
@@ -298,6 +306,42 @@ def run_model(planes_nhwc, dec, coords, box_warp, impl=None, sigma_only=False):
             _lib.check(st, 'p3d_run_model')
     _lib.bump()
     return rgb, sigma
+
+
+def marching_cubes(volume, threshold):
+    """Marching cubes (p3d_marching_cubes_*, the mesh of include/p3d.h) on a float32 CUDA grid [nx,ny,nz], each side >= 2:
+    -> (vertices float64 [V,3] in index coordinates, faces int64 [F,3]) on the volume's device.
+
+    The output size is known only after the count, so this reads the two counts back once (one synchronisation of the
+    current stream) before it allocates the outputs; it cannot be captured in a CUDA graph. Refuses V >= 2^31."""
+    if volume.dim() != 3 or min(volume.shape) < 2:
+        raise ValueError(f'volume must be [nx,ny,nz] with every side >= 2, got {tuple(volume.shape)}')
+    if volume.dtype != torch.float32 or not volume.is_cuda:
+        raise TypeError(f'volume must be a float32 CUDA tensor, got {volume.dtype} on {volume.device}')
+    v = volume.contiguous()
+    nx, ny, nz = v.shape
+    dev = v.device
+    lib = _lib.lib()
+    ws_bytes = lib.p3d_marching_cubes_workspace_bytes(nx, ny, nz)
+    if ws_bytes < 0:
+        raise ValueError(f'grid {tuple(v.shape)} is too large for p3d_marching_cubes')
+    ws = torch.empty(ws_bytes, device=dev, dtype=torch.uint8)
+    counts = torch.empty(2, device=dev, dtype=torch.int64)
+    thr = ctypes.c_double(float(threshold))
+    with torch.cuda.device(dev):
+        _lib.check(lib.p3d_marching_cubes_count(_lib.ptr(v), nx, ny, nz, thr, _lib.ptr(ws), ws_bytes, _lib.ptr(counts),
+                                                _lib.stream_ptr()), 'p3d_marching_cubes_count')
+        _lib.bump(2)
+        n_verts, n_faces = counts.tolist()
+        if n_verts >= 1 << 31:
+            raise ValueError(f'{n_verts} vertices: p3d_marching_cubes supports fewer than 2^31')
+        vertices = torch.empty(n_verts, 3, device=dev, dtype=torch.float64)
+        faces = torch.empty(n_faces, 3, device=dev, dtype=torch.int64)
+        if n_verts:
+            _lib.check(lib.p3d_marching_cubes_emit(_lib.ptr(v), nx, ny, nz, thr, _lib.ptr(ws), ws_bytes, _lib.ptr(vertices),
+                                                   _lib.ptr(faces), _lib.stream_ptr()), 'p3d_marching_cubes_emit')
+            _lib.bump(2)
+    return vertices, faces
 
 
 def sample_from_planes(planes_nhwc, coords, box_warp):

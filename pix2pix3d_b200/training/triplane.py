@@ -88,10 +88,15 @@ def _sr_kwargs(synthesis_kwargs):
     return {k: v for k, v in synthesis_kwargs.items() if k != 'noise_mode'}
 
 
+def query_planes(gen, ws, update_emas, synthesis_kwargs):
+    """The tri-planes [B,3,32,H,W] that `query_points` queries (also used by pix2pix3d_b200.mesh.sigma_grid)."""
+    planes = gen.backbone.synthesis(ws, update_emas=update_emas, **synthesis_kwargs)
+    return planes.view(len(planes), 3, 32, planes.shape[-2], planes.shape[-1])
+
+
 def query_points(gen, coordinates, directions, ws, update_emas, synthesis_kwargs):
     """Backbone + `renderer.run_model` at arbitrary 3-D points (reference triplane_cond.py:1070-1074)."""
-    planes = gen.backbone.synthesis(ws, update_emas=update_emas, **synthesis_kwargs)
-    planes = planes.view(len(planes), 3, 32, planes.shape[-2], planes.shape[-1])
+    planes = query_planes(gen, ws, update_emas, synthesis_kwargs)
     return gen.renderer.run_model(planes, gen.decoder, coordinates, directions, gen.rendering_kwargs)
 
 
