@@ -489,6 +489,57 @@ int p3d_marching_cubes_count(const float* volume, int64_t nx, int64_t ny, int64_
 int p3d_marching_cubes_emit(const float* volume, int64_t nx, int64_t ny, int64_t nz, double threshold,
                             void* workspace, int64_t workspace_bytes, double* vertices, int64_t* faces, p3d_stream_t stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Mesh preview (applications/extract_mesh.py:226-262: the pyrender turntable of the extracted mesh)
+ *
+ * A triangle rasterizer with a depth buffer and a diffuse shader (pix2pix3d_b200/csrc/mesh_raster.cu; the numpy
+ * restatement is oracle/p3d_oracle/mesh_render.py). It is not pyrender and does not reproduce its pixels.
+ * From the script: the orthographic camera and its extents (xmag = ymag = 0.3 for seg, 0.6 for car), the 512x512 frames,
+ * the orbit of OpenGL-convention poses and a spot light of intensity 3 with a pi/4 cone placed at the camera.
+ * This package's choices: diffuse shading only (no ambient, no specular), a hard cone edge, grey 0.8 when the mesh has
+ * no vertex colours, a white background, and znear = 0.05 / zfar = 100 (pyrender's own defaults for the planes, the
+ * outer cone and the background are unverified).
+ *
+ * Views: per view, world2cam rows 0-2 of the inverse of an OpenGL cam2world (camera looks down -z, +y is up), the eye
+ * (camera position) and the spot axis (the camera's -z in world space), all fp32.
+ * Every product and sum below is one fp32 operation rounded to nearest, in the order written (no FMA contraction):
+ *   c = ((m[r][0] x + m[r][1] y) + m[r][2] z) + m[r][3]       camera coordinates, r = 0, 1, 2
+ *   sx = c0 (W / (2 xmag)) + W / 2,  sy = H / 2 - c1 (H / (2 ymag)),  d = -c2      (row 0 is the top)
+ * Coverage: X = rint(256 sx), Y = rint(256 sy) (int64, 8 sub-pixel bits). Pixel (i, j) has its centre at
+ * (256 j + 128, 256 i + 128). Edge functions E_k (edge opposite vertex k, from vertex k+1 to k+2) are exact integers and
+ * sum to the area A. A triangle with A < 0 has every E_k and A negated (either winding is drawn); A == 0 is skipped.
+ * A pixel is covered when every E_k > 0, or E_k == 0 on a top-left edge (edge vector (dx, dy) after the negation:
+ * dy < 0, or dy == 0 and dx > 0), so two triangles sharing an edge cover each pixel on it exactly once.
+ * Dropped triangles: a non-finite vertex coordinate or a face index outside [0, V) (silently: marching cubes emits NaN
+ * vertices next to NaN grid values), and a vertex with |sx| or |sy| not <= 2^21 (counted into guard_drops[0]).
+ * Depth: b_k = fp32(E_k) / fp32(A) (correctly rounded conversions), d = (b0 d0 + b1 d1) + b2 d2; a fragment is kept when
+ * znear <= d <= zfar. depth_keys [N,H,W] = min over fragments of (float_bits(d) << 32 | face id): the nearest fragment
+ * wins, the lower face id on equal depth, whatever the launch order; ~0 = empty.
+ * Shading, per covered pixel, with the same b_k, world vertices v_k and colours c_k (uint8 / 255 or grey 0.8):
+ *   colour = (b0 c0 + b1 c1) + b2 c2 per channel;  n = cross(v1 - v0, v2 - v0) / |.|  (outward for marching_cubes faces);
+ *   p = (b0 v0 + b1 v1) + b2 v2;  q = eye - p;  r2 = (qx qx + qy qy) + qz qz;  l = q / sqrt(r2);
+ *   shade = (I max(0, n . l)) / (pi r2), or 0 when (axis . l) > -cos(pi/4) (outside the cone);
+ *   out = x < 255 ? floor(x) : 255 with x = ((255 colour) shade) + 0.5; empty pixels are white (255, 255, 255).
+ * Vector lengths are sqrt of (x x + y y) + z z and divisions are correctly rounded (no reciprocal square roots). */
+typedef struct {
+    float world2cam[12];     /* rows 0-2 of the 4x4 world-to-camera matrix, row-major */
+    float eye[3];            /* camera position in world space (where the light sits) */
+    float spot_axis[3];      /* camera -z in world space */
+} p3d_mesh_view_t;
+
+/* Depth pass: vertices [V,3] fp32, faces [F,3] int64 (what p3d_marching_cubes_emit writes), views [N] (device array),
+ * depth_keys uint64 [N,H,W] (cleared to ~0 here), guard_drops: one device int64 (zeroed here, then the number of
+ * (face, view) pairs dropped by the guard band). One launch covers every face and view. P3D_BAD_ARG on bad sizes
+ * (N, H or W < 1, F >= 2^32, xmag / ymag not > 0, not 0 < znear < zfar). */
+int p3d_mesh_raster(const float* vertices, int64_t V, const int64_t* faces, int64_t F, const p3d_mesh_view_t* views, int N,
+                    int H, int W, float xmag, float ymag, float znear, float zfar, uint64_t* depth_keys, int64_t* guard_drops,
+                    p3d_stream_t stream);
+/* Shading pass over the keys of p3d_mesh_raster (same vertices, faces, views and extents): out uint8 [N,H,W,3].
+ * vertex_colors: uint8 [V,3] or NULL (grey). light_intensity: I above. */
+int p3d_mesh_shade(const uint64_t* depth_keys, const float* vertices, int64_t V, const int64_t* faces, int64_t F,
+                   const p3d_mesh_view_t* views, int N, int H, int W, float xmag, float ymag,
+                   const unsigned char* vertex_colors, float light_intensity, unsigned char* out, p3d_stream_t stream);
+
 /* upsample2d(img, f) with up=2 (upfirdn2d.py:315-350) on an fp32 NHWC image: [B,H,W,C] -> [B,2H,2W,C]. */
 int p3d_upsample2x_nhwc(const float* x, const float* f, float* y, int B, int H, int W, int C, p3d_stream_t stream);
 

@@ -10,7 +10,7 @@ import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'libp3d.so')
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 _lib = None
 
@@ -58,6 +58,8 @@ class FilteredLReluArgs(ctypes.Structure):  # p3d_filtered_lrelu_args_t
         ('b_stride', c_int64), ('s_shape', c_int32 * 2), ('s_ofs', c_int32 * 2), ('sw_limit', c_int32), ('sign_mode', c_int32),
     ]
 
+
+MESH_VIEW_FLOATS = 18    # p3d_mesh_view_t: world2cam rows 0-2 (12), eye (3), spot axis (3)
 
 _SIGNATURES = {
     'p3d_abi_version': (c_int, []),
@@ -129,6 +131,10 @@ _SIGNATURES = {
                                          c_void_p]),
     'p3d_marching_cubes_emit': (c_int, [c_void_p, c_int64, c_int64, c_int64, ctypes.c_double, c_void_p, c_int64, c_void_p,
                                         c_void_p, c_void_p]),
+    'p3d_mesh_raster': (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int, c_int, c_int, c_float, c_float, c_float,
+                                c_float, c_void_p, c_void_p, c_void_p]),
+    'p3d_mesh_shade': (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int, c_int, c_int, c_float, c_float,
+                               c_void_p, c_float, c_void_p, c_void_p]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

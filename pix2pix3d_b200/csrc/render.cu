@@ -736,7 +736,7 @@ using namespace p3d;
 
 extern "C" {
 
-int p3d_abi_version(void) { return 6; }
+int p3d_abi_version(void) { return 7; }
 const char* p3d_build_info(void) { return "libp3d sm_100a " __DATE__ " " __TIME__; }
 const char* p3d_status_string(int status) {
     if (status == P3D_OK) return "ok";

@@ -344,6 +344,72 @@ def marching_cubes(volume, threshold):
     return vertices, faces
 
 
+def mesh_views(cam2world_gl):
+    """p3d_mesh_view_t array of OpenGL-convention poses [N,4,4] (camera looks down -z, +y up): float32 CPU tensor
+    [N,18] = world2cam rows 0-2, eye, spot axis (camera -z). The rigid inverse (R^T, -R^T t) is formed in float64 and cast
+    to float32 once."""
+    c = cam2world_gl.detach().cpu().double().numpy() if isinstance(cam2world_gl, torch.Tensor) else np.asarray(cam2world_gl, np.float64)
+    c = c.reshape(-1, 4, 4)
+    R, t = c[:, :3, :3], c[:, :3, 3]
+    Rt = R.transpose(0, 2, 1)
+    w2c = np.concatenate([Rt, -np.einsum('nij,nj->ni', Rt, t)[:, :, None]], 2)
+    views = np.concatenate([w2c.reshape(-1, 12), t, -R[:, :, 2]], 1).astype(np.float32)
+    return torch.from_numpy(np.ascontiguousarray(views))
+
+
+def _mesh_inputs(vertices, faces, views):
+    if not (vertices.is_cuda and vertices.dtype == torch.float32 and vertices.dim() == 2 and vertices.shape[1] == 3):
+        raise TypeError(f'vertices must be a float32 CUDA tensor [V,3], got {vertices.dtype} {tuple(vertices.shape)} on {vertices.device}')
+    if not (faces.dtype == torch.int64 and faces.dim() == 2 and faces.shape[1] == 3 and faces.device == vertices.device):
+        raise TypeError(f'faces must be an int64 tensor [F,3] on {vertices.device}, got {faces.dtype} {tuple(faces.shape)} on {faces.device}')
+    if not (views.dtype == torch.float32 and views.dim() == 2 and views.shape[1] == _lib.MESH_VIEW_FLOATS
+            and views.device == vertices.device):
+        raise TypeError(f'views must be float32 [N,{_lib.MESH_VIEW_FLOATS}] on {vertices.device} (mesh_views)')
+    return vertices.contiguous(), faces.contiguous(), views.contiguous()
+
+
+def mesh_raster(vertices, faces, views, height, width, xmag, ymag, znear, zfar):
+    """Depth pass of the mesh preview (p3d_mesh_raster; contract in include/p3d.h): vertices float32 CUDA [V,3], faces int64
+    [F,3], views float32 [N,18] (mesh_views) -> depth keys [N,H,W] (int64 tensor holding the uint64 keys; -1 = empty).
+    Reads the guard-band drop count back (one synchronisation) and raises ValueError when a triangle left the guard band."""
+    v, f, views = _mesh_inputs(vertices, faces, views)
+    N, dev = views.shape[0], v.device
+    keys = torch.empty(N, height, width, device=dev, dtype=torch.int64)
+    drops = torch.empty(1, device=dev, dtype=torch.int64)
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib().p3d_mesh_raster(_lib.ptr(v), v.shape[0], _lib.ptr(f), f.shape[0], _lib.ptr(views), N, height, width,
+                                              float(xmag), float(ymag), float(znear), float(zfar), _lib.ptr(keys), _lib.ptr(drops),
+                                              _lib.stream_ptr()), 'p3d_mesh_raster')
+        _lib.bump()
+        n_drop = int(drops.item())
+    if n_drop:
+        raise ValueError(f'{n_drop} (triangle, view) pairs have a vertex more than 2^21 pixels off screen; '
+                         'move the camera or scale the mesh')
+    return keys
+
+
+def mesh_shade(keys, vertices, faces, views, xmag, ymag, vertex_colors=None, light_intensity=3.0):
+    """Shading pass of the mesh preview (p3d_mesh_shade) over the keys of mesh_raster -> uint8 [N,H,W,3].
+    vertex_colors: uint8 [V,3] on the vertices' device, or None (grey)."""
+    v, f, views = _mesh_inputs(vertices, faces, views)
+    N, H, W = keys.shape
+    if keys.dtype != torch.int64 or keys.device != v.device or N != views.shape[0]:
+        raise TypeError('keys must be the int64 [N,H,W] output of mesh_raster for these views')
+    keys = keys.contiguous()
+    col = None
+    if vertex_colors is not None:
+        if not (vertex_colors.dtype == torch.uint8 and tuple(vertex_colors.shape) == (v.shape[0], 3) and vertex_colors.device == v.device):
+            raise TypeError(f'vertex_colors must be uint8 [{v.shape[0]},3] on {v.device}')
+        col = vertex_colors.contiguous()
+    out = torch.empty(N, H, W, 3, device=v.device, dtype=torch.uint8)
+    with torch.cuda.device(v.device):
+        _lib.check(_lib.lib().p3d_mesh_shade(_lib.ptr(keys), _lib.ptr(v), v.shape[0], _lib.ptr(f), f.shape[0], _lib.ptr(views), N, H, W,
+                                             float(xmag), float(ymag), _lib.ptr(col), float(light_intensity), _lib.ptr(out),
+                                             _lib.stream_ptr()), 'p3d_mesh_shade')
+    _lib.bump()
+    return out
+
+
 def sample_from_planes(planes_nhwc, coords, box_warp):
     """coords [B,M,3] -> features [B,3,M,32] (reference layout of sample_from_planes)."""
     B, _, H, W, _ = planes_nhwc.shape
