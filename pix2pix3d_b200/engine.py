@@ -19,7 +19,7 @@ import weakref
 import numpy as np
 import torch
 
-from . import tcconv
+from . import _lib, tcconv
 
 _SQRT2 = float(np.sqrt(2))
 
@@ -200,7 +200,7 @@ class WeightPlan(StylePlan):
     def tables(self, b):
         t = self._tables.get(b)
         if t is None:
-            descs = (tcconv.ModwDesc * len(self.specs))()
+            descs = (_lib.ModwDesc * len(self.specs))()
             block_layer, out_off, styles_off, first = [], 0, 0, 0
             shapes = []
             for k, (sp, (wt, wsq), n_in) in enumerate(zip(self.specs, self.prepared, self.sizes)):

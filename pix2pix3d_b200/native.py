@@ -17,11 +17,26 @@ TC_PACKED_BYTES = 65536 + 324 * 4
 # 'tc_pairs' (tensor-core decoder, ray-pair ownership: render_tc2.cu; sample counts <= 64)
 render_impl = 'auto'
 
-# when set to a list, render_fwd appends ('render_fwd', start_event, end_event) around its launch (bench.py)
+# when set to a list, timed_call records its launches here: ('render_fwd', start_event, end_event) from render_fwd and
+# ('conv_gemm', start_event, end_event, flops, executed_flops) from the tcconv convolutions (bench.py)
 kernel_events = None
 # when set to a dict, every render_fwd call also writes the kernel's bookkeeping (importance indices, fine depths, sort
 # permutation, interval weights) and leaves it there: lets tests score the bookkeeping of a whole G.synthesis call
 render_debug_sink = None
+
+
+def timed_call(event, name, *args, device, unsupported_ok=False):
+    """_lib.call; with kernel_events set, a launch that ran is bracketed by CUDA events and recorded as
+    (event[0], start, end, *event[1:])."""
+    if kernel_events is None:
+        return _lib.call(name, *args, device=device, unsupported_ok=unsupported_ok)
+    start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    start.record()
+    ran = _lib.call(name, *args, device=device, unsupported_ok=unsupported_ok)
+    if ran:
+        end.record()
+        kernel_events.append((event[0], start, end, *event[1:]))
+    return ran
 
 
 def _f32c(t):
@@ -39,11 +54,7 @@ def ray_sampler(cam2world, intrinsics, resolution):
     M = resolution * resolution
     origins = torch.empty(B, M, 3, device=c2w.device, dtype=torch.float32)
     dirs = torch.empty_like(origins)
-    with torch.cuda.device(c2w.device):
-        st = _lib.lib().p3d_ray_sampler(_lib.ptr(c2w), _lib.ptr(K), B, resolution, _lib.ptr(origins), _lib.ptr(dirs),
-                                        _lib.stream_ptr())
-    _lib.check(st, 'p3d_ray_sampler')
-    _lib.bump()
+    _lib.call('p3d_ray_sampler', c2w, K, B, resolution, origins, dirs, device=c2w.device)
     return origins, dirs
 
 
@@ -54,10 +65,7 @@ def planes_to_channels_last(planes):
     C, H, W = shp[-3], shp[-2], shp[-1]
     N = p.numel() // (C * H * W)
     out = torch.empty(*shp[:-3], H, W, C, device=p.device, dtype=torch.float32)
-    with torch.cuda.device(p.device):
-        st = _lib.lib().p3d_planes_to_channels_last(_lib.ptr(p), _lib.ptr(out), N, C, H, W, _lib.stream_ptr())
-    _lib.check(st, 'p3d_planes_to_channels_last')
-    _lib.bump()
+    _lib.call('p3d_planes_to_channels_last', p, out, N, C, H, W, device=p.device)
     return out
 
 
@@ -123,14 +131,9 @@ def pack_decoder(decoder):
         d.w2_gain[i], d.b2_gain[i] = float(fc2.weight_gain), float(fc2.bias_gain)
         d.sigmoid_mask[i] = masks[i]
     packed = torch.empty(PACKED_FLOATS, device=dev, dtype=torch.float32)
-    with torch.cuda.device(dev):
-        st = _lib.lib().p3d_pack_decoder(ctypes.byref(d), _lib.ptr(packed), _lib.stream_ptr())
-    _lib.check(st, 'p3d_pack_decoder')
+    _lib.call('p3d_pack_decoder', ctypes.byref(d), packed, device=dev)
     packed_tc = torch.empty(TC_PACKED_BYTES, device=dev, dtype=torch.uint8)
-    with torch.cuda.device(dev):
-        st = _lib.lib().p3d_pack_decoder_tc(ctypes.byref(d), _lib.ptr(packed_tc), _lib.stream_ptr())
-    _lib.check(st, 'p3d_pack_decoder_tc')
-    _lib.bump(2)
+    _lib.call('p3d_pack_decoder_tc', ctypes.byref(d), packed_tc, device=dev)
     del keep
     return PackedDecoder(packed, len(nets), sigma_net, masks, packed_tc)
 
@@ -142,10 +145,7 @@ def ray_limits_box(rays_o, rays_d, box_side_length):
     n = o.shape[0]
     tn = torch.empty(n, device=o.device, dtype=torch.float32)
     tf = torch.empty(n, device=o.device, dtype=torch.float32)
-    with torch.cuda.device(o.device):
-        st = _lib.lib().p3d_ray_limits_box(_lib.ptr(o), _lib.ptr(d), n, float(box_side_length), _lib.ptr(tn), _lib.ptr(tf), _lib.stream_ptr())
-    _lib.check(st, 'p3d_ray_limits_box')
-    _lib.bump()
+    _lib.call('p3d_ray_limits_box', o, d, n, float(box_side_length), tn, tf, device=o.device)
     return tn.reshape(*lead, 1), tf.reshape(*lead, 1)
 
 
@@ -230,31 +230,19 @@ def render_fwd(planes_nhwc, dec, ray_origins, ray_dirs, depths_coarse, u, box_wa
     a.workspace = ws.data_ptr()
     if strided:
         a.plane_strides[0], a.plane_strides[1], a.plane_strides[2] = st_img, st_plane, st_pix
-    ev = None
-    if kernel_events is not None:
-        ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
-        ev[0].record()
     use_tc = impl in ('auto', 'tc', 'tc_pairs') and Sc % 8 == 0 and Sf % 8 == 0 and Sc <= 128 and Sf <= 128 and dec.packed_tc is not None
     if impl in ('tc', 'tc_pairs') and not use_tc:
         raise ValueError('tensor-core renderer needs sample counts that are multiples of 8')
     # ray-pair ownership fills its rows only at 64 samples per pass; there it is 6-8 % faster (1.58 vs 1.72 ms at the config-4
     # sampling), at 48 it is 21 % slower (profiles/r01_render_fwd_tc_ncu.md)
     a.tc_variant = 1 if (impl == 'tc_pairs' or (impl == 'auto' and Sc == 64 and Sf == 64)) else 0
-    with torch.cuda.device(dev):
-        if use_tc:
-            a.decoder_packed = dec.packed_tc.data_ptr()
-            st = _lib.lib().p3d_render_fwd_tc(ctypes.byref(a), _lib.stream_ptr())
-        else:
-            if strided:   # the SIMT kernel reads dense planes only
-                dense = planes_nhwc.contiguous()
-                a.planes_nhwc = dense.data_ptr()
-                a.plane_strides[0] = a.plane_strides[1] = a.plane_strides[2] = 0
-            st = _lib.lib().p3d_render_fwd(ctypes.byref(a), _lib.stream_ptr())
-    if ev is not None:
-        ev[1].record()
-        kernel_events.append(('render_fwd', ev[0], ev[1]))
-    _lib.check(st, 'p3d_render_fwd')
-    _lib.bump()
+    if use_tc:
+        a.decoder_packed = dec.packed_tc.data_ptr()
+    elif strided:   # the SIMT kernel reads dense planes only
+        dense = planes_nhwc.contiguous()
+        a.planes_nhwc = dense.data_ptr()
+        a.plane_strides[0] = a.plane_strides[1] = a.plane_strides[2] = 0
+    timed_call(('render_fwd',), 'p3d_render_fwd_tc' if use_tc else 'p3d_render_fwd', ctypes.byref(a), device=dev)
     if render_debug_sink is not None:
         render_debug_sink.update(dbg, feat=feat, depth=depth, wsum=wsum)
     if debug:
@@ -293,18 +281,12 @@ def run_model(planes_nhwc, dec, coords, box_warp, impl=None, sigma_only=False, o
             raise ValueError(f'out_sigma must be a contiguous float32 tensor of {B * M} elements on {dev}')
         sigma = out_sigma
     masks = (ctypes.c_uint32 * 2)(dec.masks[0], dec.masks[1])
-    with torch.cuda.device(dev):
-        if use_tc:
-            st = _lib.lib().p3d_run_model_tc(_lib.ptr(planes_nhwc), strides, _lib.ptr(c), _lib.ptr(dec.packed_tc), dec.n_nets,
-                                             dec.sigma_net, masks, B, M, H, W, 2.0 / float(box_warp), _lib.ptr(rgb),
-                                             _lib.ptr(sigma), _lib.stream_ptr())
-            _lib.check(st, 'p3d_run_model_tc')
-        else:
-            st = _lib.lib().p3d_run_model(_lib.ptr(planes_nhwc), _lib.ptr(c), _lib.ptr(dec.packed), dec.n_nets, dec.sigma_net,
-                                          masks, B, M, H, W, 2.0 / float(box_warp), _lib.ptr(rgb), _lib.ptr(sigma),
-                                          _lib.stream_ptr())
-            _lib.check(st, 'p3d_run_model')
-    _lib.bump()
+    if use_tc:
+        _lib.call('p3d_run_model_tc', planes_nhwc, strides, c, dec.packed_tc, dec.n_nets, dec.sigma_net, masks, B, M, H, W,
+                  2.0 / float(box_warp), rgb, sigma, device=dev)
+    else:
+        _lib.call('p3d_run_model', planes_nhwc, c, dec.packed, dec.n_nets, dec.sigma_net, masks, B, M, H, W, 2.0 / float(box_warp),
+                  rgb, sigma, device=dev)
     return rgb, sigma
 
 
@@ -321,26 +303,20 @@ def marching_cubes(volume, threshold):
     v = volume.contiguous()
     nx, ny, nz = v.shape
     dev = v.device
-    lib = _lib.lib()
-    ws_bytes = lib.p3d_marching_cubes_workspace_bytes(nx, ny, nz)
+    ws_bytes = _lib.lib().p3d_marching_cubes_workspace_bytes(nx, ny, nz)
     if ws_bytes < 0:
         raise ValueError(f'grid {tuple(v.shape)} is too large for p3d_marching_cubes')
     ws = torch.empty(ws_bytes, device=dev, dtype=torch.uint8)
     counts = torch.empty(2, device=dev, dtype=torch.int64)
     thr = ctypes.c_double(float(threshold))
-    with torch.cuda.device(dev):
-        _lib.check(lib.p3d_marching_cubes_count(_lib.ptr(v), nx, ny, nz, thr, _lib.ptr(ws), ws_bytes, _lib.ptr(counts),
-                                                _lib.stream_ptr()), 'p3d_marching_cubes_count')
-        _lib.bump(2)
-        n_verts, n_faces = counts.tolist()
-        if n_verts >= 1 << 31:
-            raise ValueError(f'{n_verts} vertices: p3d_marching_cubes supports fewer than 2^31')
-        vertices = torch.empty(n_verts, 3, device=dev, dtype=torch.float64)
-        faces = torch.empty(n_faces, 3, device=dev, dtype=torch.int64)
-        if n_verts:
-            _lib.check(lib.p3d_marching_cubes_emit(_lib.ptr(v), nx, ny, nz, thr, _lib.ptr(ws), ws_bytes, _lib.ptr(vertices),
-                                                   _lib.ptr(faces), _lib.stream_ptr()), 'p3d_marching_cubes_emit')
-            _lib.bump(2)
+    _lib.call('p3d_marching_cubes_count', v, nx, ny, nz, thr, ws, ws_bytes, counts, device=dev)
+    n_verts, n_faces = counts.tolist()
+    if n_verts >= 1 << 31:
+        raise ValueError(f'{n_verts} vertices: p3d_marching_cubes supports fewer than 2^31')
+    vertices = torch.empty(n_verts, 3, device=dev, dtype=torch.float64)
+    faces = torch.empty(n_faces, 3, device=dev, dtype=torch.int64)
+    if n_verts:
+        _lib.call('p3d_marching_cubes_emit', v, nx, ny, nz, thr, ws, ws_bytes, vertices, faces, device=dev)
     return vertices, faces
 
 
@@ -376,12 +352,9 @@ def mesh_raster(vertices, faces, views, height, width, xmag, ymag, znear, zfar):
     N, dev = views.shape[0], v.device
     keys = torch.empty(N, height, width, device=dev, dtype=torch.int64)
     drops = torch.empty(1, device=dev, dtype=torch.int64)
-    with torch.cuda.device(dev):
-        _lib.check(_lib.lib().p3d_mesh_raster(_lib.ptr(v), v.shape[0], _lib.ptr(f), f.shape[0], _lib.ptr(views), N, height, width,
-                                              float(xmag), float(ymag), float(znear), float(zfar), _lib.ptr(keys), _lib.ptr(drops),
-                                              _lib.stream_ptr()), 'p3d_mesh_raster')
-        _lib.bump()
-        n_drop = int(drops.item())
+    _lib.call('p3d_mesh_raster', v, v.shape[0], f, f.shape[0], views, N, height, width, float(xmag), float(ymag), float(znear),
+              float(zfar), keys, drops, device=dev)
+    n_drop = int(drops.item())
     if n_drop:
         raise ValueError(f'{n_drop} (triangle, view) pairs have a vertex more than 2^21 pixels off screen; '
                          'move the camera or scale the mesh')
@@ -402,11 +375,8 @@ def mesh_shade(keys, vertices, faces, views, xmag, ymag, vertex_colors=None, lig
             raise TypeError(f'vertex_colors must be uint8 [{v.shape[0]},3] on {v.device}')
         col = vertex_colors.contiguous()
     out = torch.empty(N, H, W, 3, device=v.device, dtype=torch.uint8)
-    with torch.cuda.device(v.device):
-        _lib.check(_lib.lib().p3d_mesh_shade(_lib.ptr(keys), _lib.ptr(v), v.shape[0], _lib.ptr(f), f.shape[0], _lib.ptr(views), N, H, W,
-                                             float(xmag), float(ymag), _lib.ptr(col), float(light_intensity), _lib.ptr(out),
-                                             _lib.stream_ptr()), 'p3d_mesh_shade')
-    _lib.bump()
+    _lib.call('p3d_mesh_shade', keys, v, v.shape[0], f, f.shape[0], views, N, H, W, float(xmag), float(ymag), col,
+              float(light_intensity), out, device=v.device)
     return out
 
 
@@ -416,11 +386,7 @@ def sample_from_planes(planes_nhwc, coords, box_warp):
     c = _f32c(coords)
     M = c.shape[1]
     out = torch.empty(B, 3, M, 32, device=planes_nhwc.device, dtype=torch.float32)
-    with torch.cuda.device(planes_nhwc.device):
-        st = _lib.lib().p3d_sample_from_planes(_lib.ptr(planes_nhwc), _lib.ptr(c), B, M, H, W, 2.0 / float(box_warp),
-                                               _lib.ptr(out), _lib.stream_ptr())
-    _lib.check(st, 'p3d_sample_from_planes')
-    _lib.bump()
+    _lib.call('p3d_sample_from_planes', planes_nhwc, c, B, M, H, W, 2.0 / float(box_warp), out, device=planes_nhwc.device)
     return out
 
 
@@ -433,11 +399,7 @@ def ray_march(colors, densities, depths, white_back=False):
     depth = torch.empty(B, R, 1, device=dev, dtype=torch.float32)
     weights = torch.empty(B, R, S - 1, 1, device=dev, dtype=torch.float32)
     ws = torch.empty(4, device=dev, dtype=torch.int32)
-    with torch.cuda.device(dev):
-        st = _lib.lib().p3d_ray_march(_lib.ptr(col), _lib.ptr(den), _lib.ptr(dep), B * R, S, Cc, 1 if white_back else 0,
-                                      _lib.ptr(rgb), _lib.ptr(depth), _lib.ptr(weights), _lib.ptr(ws), _lib.stream_ptr())
-    _lib.check(st, 'p3d_ray_march')
-    _lib.bump()
+    _lib.call('p3d_ray_march', col, den, dep, B * R, S, Cc, 1 if white_back else 0, rgb, depth, weights, ws, device=dev)
     return rgb, depth, weights
 
 
@@ -447,11 +409,7 @@ def sample_from_planes_bwd(grad_features, coords, box_warp, H, W):
     c = _f32c(coords)
     B, _, M, _ = g.shape
     out = torch.empty(B, 3, H, W, 32, device=g.device, dtype=torch.float32)
-    with torch.cuda.device(g.device):
-        st = _lib.lib().p3d_sample_from_planes_bwd(_lib.ptr(g), _lib.ptr(c), B, M, H, W, 2.0 / float(box_warp), _lib.ptr(out),
-                                                   _lib.stream_ptr())
-    _lib.check(st, 'p3d_sample_from_planes_bwd')
-    _lib.bump()
+    _lib.call('p3d_sample_from_planes_bwd', g, c, B, M, H, W, 2.0 / float(box_warp), out, device=g.device)
     return out
 
 
@@ -465,12 +423,8 @@ def ray_march_bwd(colors, densities, depths, g_rgb, g_depth, g_weights, depth_ra
     rng = None if depth_range is None else _f32c(depth_range)
     g_col = torch.empty_like(col)
     g_den = torch.empty_like(den)
-    with torch.cuda.device(col.device):
-        st = _lib.lib().p3d_ray_march_bwd(_lib.ptr(col), _lib.ptr(den), _lib.ptr(dep), _lib.ptr(grgb), _lib.ptr(gdep),
-                                          _lib.ptr(gw), _lib.ptr(rng), B * R, S, Cc, 1 if white_back else 0, _lib.ptr(g_col),
-                                          _lib.ptr(g_den), _lib.stream_ptr())
-    _lib.check(st, 'p3d_ray_march_bwd')
-    _lib.bump()
+    _lib.call('p3d_ray_march_bwd', col, den, dep, grgb, gdep, gw, rng, B * R, S, Cc, 1 if white_back else 0, g_col, g_den,
+              device=col.device)
     return g_col, g_den
 
 
@@ -481,11 +435,7 @@ def sample_importance(z_vals, weights, u, return_inds=False):
     Sf = uu.shape[1]
     out = torch.empty(N, Sf, device=z.device, dtype=torch.float32)
     inds = torch.empty(N, Sf, device=z.device, dtype=torch.int32) if return_inds else None
-    with torch.cuda.device(z.device):
-        st = _lib.lib().p3d_sample_importance(_lib.ptr(z), _lib.ptr(w), _lib.ptr(uu), N, S, Sf, _lib.ptr(out),
-                                              _lib.ptr(inds), _lib.stream_ptr())
-    _lib.check(st, 'p3d_sample_importance')
-    _lib.bump()
+    _lib.call('p3d_sample_importance', z, w, uu, N, S, Sf, out, inds, device=z.device)
     return (out, inds) if return_inds else out
 
 
@@ -508,11 +458,7 @@ class _DecoderMLP(torch.autograd.Function):
         sigma = torch.empty(n, m, 1, device=f.device, dtype=torch.float32)
         # hidden pre-activations for the backward pass (256 bytes per point), only when a gradient can be asked for
         pre = torch.empty(n * m, 64, device=f.device, dtype=torch.float32) if any(ctx.needs_input_grad) else None
-        with torch.cuda.device(f.device):
-            st = _lib.lib().p3d_decoder_mlp_fwd(_lib.ptr(f), n, m, _lib.ptr(w1c), _lib.ptr(b1c), _lib.ptr(w2c), _lib.ptr(b2c), int(mask),
-                                                _lib.ptr(rgb), _lib.ptr(sigma), _lib.ptr(pre), _lib.stream_ptr())
-        _lib.check(st, 'p3d_decoder_mlp_fwd')
-        _lib.bump()
+        _lib.call('p3d_decoder_mlp_fwd', f, n, m, w1c, b1c, w2c, b2c, int(mask), rgb, sigma, pre, device=f.device)
         if pre is not None:
             ctx.save_for_backward(f, w1c, b1c, w2c, b2c, pre, rgb)
         ctx.mask = int(mask)
@@ -527,14 +473,10 @@ class _DecoderMLP(torch.autograd.Function):
         gs = None if g_sigma is None else _f32c(g_sigma)
         g_feats = torch.empty_like(f)
         g_params = torch.empty(DECODER_PARAM_FLOATS, device=f.device, dtype=torch.float32)
-        with torch.cuda.device(f.device):
-            nws = _lib.lib().p3d_decoder_mlp_bwd_workspace_floats()
-            ws = torch.empty(nws, device=f.device, dtype=torch.float32)
-            st = _lib.lib().p3d_decoder_mlp_bwd(_lib.ptr(f), _lib.ptr(pre), _lib.ptr(rgb), n, m, _lib.ptr(w1), _lib.ptr(b1), _lib.ptr(w2), _lib.ptr(b2), ctx.mask,
-                                                _lib.ptr(gr), _lib.ptr(gs), _lib.ptr(g_feats), _lib.ptr(g_params), _lib.ptr(ws), nws,
-                                                _lib.stream_ptr())
-        _lib.check(st, 'p3d_decoder_mlp_bwd')
-        _lib.bump(2)
+        nws = _lib.lib().p3d_decoder_mlp_bwd_workspace_floats()
+        ws = torch.empty(nws, device=f.device, dtype=torch.float32)
+        _lib.call('p3d_decoder_mlp_bwd', f, pre, rgb, n, m, w1, b1, w2, b2, ctx.mask, gr, gs, g_feats, g_params, ws, nws,
+                  device=f.device)
         gw1, gb1, gw2, gb2 = torch.split(g_params, [64 * 32, 64, 33 * 64, 33])
         return g_feats, gw1.view(64, 32), gb1, gw2.view(33, 64), gb2, None
 
@@ -575,9 +517,6 @@ def fc_bias_act(x, weight, bias, weight_gain, bias_gain, act, alpha, act_gain):
     xc, wc = _f32c(x.detach()), _f32c(weight.detach())
     bc = None if bias is None else _f32c(bias.detach())
     y = torch.empty(xc.shape[0], wc.shape[0], device=xc.device, dtype=torch.float32)
-    with torch.cuda.device(xc.device):
-        st = _lib.lib().p3d_fc_bias_act(_lib.ptr(xc), _lib.ptr(wc), _lib.ptr(bc), _lib.ptr(y), xc.shape[0], xc.shape[1], wc.shape[0],
-                                        float(weight_gain), float(bias_gain), int(act), float(alpha), float(act_gain), _lib.stream_ptr())
-    _lib.check(st, 'p3d_fc_bias_act')
-    _lib.bump()
+    _lib.call('p3d_fc_bias_act', xc, wc, bc, y, xc.shape[0], xc.shape[1], wc.shape[0], float(weight_gain), float(bias_gain),
+              int(act), float(alpha), float(act_gain), device=xc.device)
     return y

@@ -7,35 +7,10 @@ import os
 
 import torch
 
-from . import _lib
-
-c_int8 = ctypes.c_int8
+from . import _lib, native
+from ._lib import ConvArgs
 
 WEIGHT_SCALE = 128.0   # power of two folded into the fp16 weights so that the `lo` halves stay normal numbers
-
-
-class ConvArgs(ctypes.Structure):  # p3d_conv_args_t
-    _fields_ = [
-        ('x', ctypes.c_void_p), ('w', ctypes.c_void_p),
-        ('x_planes', ctypes.c_int32), ('w_planes', ctypes.c_int32), ('B', ctypes.c_int32), ('Bw', ctypes.c_int32),
-        ('H', ctypes.c_int32), ('W', ctypes.c_int32), ('C', ctypes.c_int32), ('Cout', ctypes.c_int32),
-        ('Cout_padded', ctypes.c_int32), ('n_kblocks', ctypes.c_int32), ('n_taps', ctypes.c_int32),
-        ('tap_dy', c_int8 * 9), ('tap_dx', c_int8 * 9), ('tap_k', c_int8 * 9),
-        ('split', ctypes.c_int32), ('gH', ctypes.c_int32), ('gW', ctypes.c_int32),
-        ('oH', ctypes.c_int32), ('oW', ctypes.c_int32), ('sy', ctypes.c_int32), ('oy', ctypes.c_int32),
-        ('sx', ctypes.c_int32), ('ox', ctypes.c_int32),
-        ('y', ctypes.c_void_p), ('y_lo', ctypes.c_void_p),
-        ('y_cstride', ctypes.c_int32), ('y_coff', ctypes.c_int32), ('out_mode', ctypes.c_int32),
-        ('bias', ctypes.c_void_p), ('noise', ctypes.c_void_p), ('dscale', ctypes.c_void_p),
-        ('act', ctypes.c_int32), ('alpha', ctypes.c_float), ('gain', ctypes.c_float), ('clamp', ctypes.c_float),
-        ('acc_scale', ctypes.c_float),
-        ('up_prev', ctypes.c_void_p), ('up_filter', ctypes.c_void_p), ('round16', ctypes.c_int32), ('out_nchw', ctypes.c_int32),
-        ('stride', ctypes.c_int32), ('launch_flags', ctypes.c_int32), ('residual', ctypes.c_void_p),
-        ('splitk_scratch', ctypes.c_void_p), ('splitk_scratch_bytes', ctypes.c_int64), ('noise_batch_stride', ctypes.c_int64),
-        ('rgb_w', ctypes.c_void_p), ('rgb_bias', ctypes.c_void_p), ('rgb_prev', ctypes.c_void_p), ('rgb_filter', ctypes.c_void_p),
-        ('rgb_out', ctypes.c_void_p), ('rgb_cout', ctypes.c_int32), ('rgb_w_rows', ctypes.c_int32), ('rgb_skip_x', ctypes.c_int32),
-        ('rgb_clamp', ctypes.c_float), ('rgb_acc_scale', ctypes.c_float),
-    ]
 
 
 # A/B switches of the convolution launcher (p3d_conv_args_t::launch_flags; results do not depend on them): bit 0 = never the
@@ -55,11 +30,7 @@ def to_nhwc_f16(x, c_padded=None, planes=1):
     n, c, h, w = x.shape
     cp = c_padded or c
     out = torch.empty(planes, n, h, w, cp, device=x.device, dtype=torch.float16)
-    with torch.cuda.device(x.device):
-        st = _lib.lib().p3d_nchw_to_nhwc_f16(_lib.ptr(x), _lib.DTYPE_CODE[x.dtype], n, c, h, w, cp, planes, _lib.ptr(out),
-                                             _lib.stream_ptr())
-    _lib.check(st, 'p3d_nchw_to_nhwc_f16')
-    _lib.bump()
+    _lib.call('p3d_nchw_to_nhwc_f16', x, _lib.DTYPE_CODE[x.dtype], n, c, h, w, cp, planes, out, device=x.device)
     return out
 
 
@@ -69,10 +40,7 @@ def nhwc_to_nchw_f32(x, channels=None, c_offset=0):
     n, h, w, cs = x.shape
     c = channels or cs
     out = torch.empty(n, c, h, w, device=x.device, dtype=torch.float32)
-    with torch.cuda.device(x.device):
-        st = _lib.lib().p3d_nhwc_to_nchw_f32(_lib.ptr(x), n, c, h, w, cs, c_offset, _lib.ptr(out), _lib.stream_ptr())
-    _lib.check(st, 'p3d_nhwc_to_nchw_f32')
-    _lib.bump()
+    _lib.call('p3d_nhwc_to_nchw_f32', x, n, c, h, w, cs, c_offset, out, device=x.device)
     return out
 
 
@@ -82,10 +50,7 @@ def prepare_weights(weight):
     o, i, kh, kw = w.shape
     wt = torch.empty(o, kh * kw, i, device=w.device, dtype=torch.float32)
     wsq = torch.empty(o, i, device=w.device, dtype=torch.float32)
-    with torch.cuda.device(w.device):
-        st = _lib.lib().p3d_prepare_weights(_lib.ptr(w), o, i, kh * kw, _lib.ptr(wt), _lib.ptr(wsq), _lib.stream_ptr())
-    _lib.check(st, 'p3d_prepare_weights')
-    _lib.bump()
+    _lib.call('p3d_prepare_weights', w, o, i, kh * kw, wt, wsq, device=w.device)
     return wt, wsq
 
 
@@ -101,38 +66,19 @@ def modulate_weights(weight, styles, demodulate=True, pre_scale=1.0, planes=1, c
     nchunk = ip // 8
     if prepared is not None and ip % 8 == 0 and nchunk <= 256 and 256 % nchunk == 0:
         wt, wsq = prepared
-        with torch.cuda.device(s.device):
-            st = _lib.lib().p3d_modulate_weights_t(_lib.ptr(wt), _lib.ptr(wsq), _lib.ptr(s), b, o, i, kh * kw, op, ip, cin_offset,
-                                                   1 if demodulate else 0, float(pre_scale), float(out_scale), planes, _lib.ptr(out),
-                                                   _lib.stream_ptr())
-        _lib.check(st, 'p3d_modulate_weights_t')
-        _lib.bump()
+        _lib.call('p3d_modulate_weights_t', wt, wsq, s, b, o, i, kh * kw, op, ip, cin_offset, 1 if demodulate else 0,
+                  float(pre_scale), float(out_scale), planes, out, device=s.device)
         return out
     w = weight.detach().float().contiguous()
-    with torch.cuda.device(w.device):
-        st = _lib.lib().p3d_modulate_weights(_lib.ptr(w), _lib.ptr(s), b, o, i, kh * kw, op, ip, cin_offset, 1 if demodulate else 0,
-                                             float(pre_scale), float(out_scale), planes, _lib.ptr(out), _lib.stream_ptr())
-    _lib.check(st, 'p3d_modulate_weights')
-    _lib.bump()
+    _lib.call('p3d_modulate_weights', w, s, b, o, i, kh * kw, op, ip, cin_offset, 1 if demodulate else 0, float(pre_scale),
+              float(out_scale), planes, out, device=w.device)
     return out
 
 
-class ModwDesc(ctypes.Structure):  # p3d_modw_desc_t
-    _fields_ = [
-        ('weight_t', ctypes.c_void_p), ('wsq', ctypes.c_void_p), ('styles_off', ctypes.c_int64), ('out_off', ctypes.c_int64),
-        ('Cout', ctypes.c_int32), ('Cin', ctypes.c_int32), ('ktaps', ctypes.c_int32), ('Cout_padded', ctypes.c_int32),
-        ('Cin_padded', ctypes.c_int32), ('cin_offset', ctypes.c_int32), ('demodulate', ctypes.c_int32), ('planes', ctypes.c_int32),
-        ('pre_scale', ctypes.c_float), ('out_scale', ctypes.c_float), ('first_block', ctypes.c_int32), ('reserved', ctypes.c_int32),
-    ]
-
-
 def modulate_weights_batch(descs_dev, block_layer_dev, n_blocks, styles_flat, out_flat, batch):
-    """One launch for every layer described by `descs_dev` (device bytes of ModwDesc[]); see p3d_modulate_weights_batch."""
-    with torch.cuda.device(styles_flat.device):
-        st = _lib.lib().p3d_modulate_weights_batch(_lib.ptr(descs_dev), _lib.ptr(block_layer_dev), n_blocks, _lib.ptr(styles_flat),
-                                                   _lib.ptr(out_flat), batch, _lib.stream_ptr())
-    _lib.check(st, 'p3d_modulate_weights_batch')
-    _lib.bump()
+    """One launch for every layer described by `descs_dev` (device bytes of _lib.ModwDesc[]); see p3d_modulate_weights_batch."""
+    _lib.call('p3d_modulate_weights_batch', descs_dev, block_layer_dev, n_blocks, styles_flat, out_flat, batch,
+              device=styles_flat.device)
 
 
 def affine_batch(ws, weight, bias, meta, out_numel):
@@ -140,11 +86,7 @@ def affine_batch(ws, weight, bias, meta, out_numel):
     ws = ws.detach().float().contiguous()
     b, num_ws, w_dim = ws.shape
     out = torch.empty(out_numel, device=ws.device, dtype=torch.float32)
-    with torch.cuda.device(ws.device):
-        st = _lib.lib().p3d_affine_batch(_lib.ptr(ws), _lib.ptr(weight), _lib.ptr(bias), _lib.ptr(meta), _lib.ptr(out), b, num_ws, w_dim,
-                                         weight.shape[0], _lib.stream_ptr())
-    _lib.check(st, 'p3d_affine_batch')
-    _lib.bump()
+    _lib.call('p3d_affine_batch', ws, weight, bias, meta, out, b, num_ws, w_dim, weight.shape[0], device=ws.device)
     return out
 
 
@@ -224,22 +166,10 @@ def _conv_args(x, w, cout, taps, grid_hw, out, out_lo=None, out_mode=0, out_map=
     return a
 
 
-def _launch(device, call, name, flops, split):
-    """Run one libp3d convolution launch; with native.kernel_events set, bracket it with CUDA events (bench.py's tensor roofline)."""
-    from . import native
-    ev = None
-    if native.kernel_events is not None:
-        ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
-        ev[0].record()
-    with torch.cuda.device(device):
-        st = call()
-    if ev is not None:
-        ev[1].record()
-        # algorithmic FLOPs of the convolution this launch implements (one pass); the fp32 layers execute 3x that on the
-        # tensor pipe (hi*hi + hi*lo + lo*hi)
-        native.kernel_events.append(('conv_gemm', ev[0], ev[1], flops, flops * (3 if split else 1)))
-    _lib.check(st, name)
-    _lib.bump()
+def _conv_event(flops, split):
+    """The native.kernel_events record of a convolution launch: `flops` are the algorithmic FLOPs of the convolution it
+    implements (one pass); the fp32 layers execute 3x that on the tensor pipe (hi*hi + hi*lo + lo*hi)."""
+    return 'conv_gemm', flops, flops * (3 if split else 1)
 
 
 def conv_gemm(x, w, cout, taps, grid_hw, out, split=False, **kw):
@@ -247,30 +177,16 @@ def conv_gemm(x, w, cout, taps, grid_hw, out, split=False, **kw):
     out: NHWC tensor [B,oH,oW,Cs] (fp16 or fp32); out_map = (sy, oy, sx, ox)."""
     a = _conv_args(x, w, cout, taps, grid_hw, out, split=split, **kw)
     flops = 2.0 * x.shape[1] * grid_hw[0] * grid_hw[1] * cout * len(taps) * x.shape[4]
-    _launch(x.device, lambda: _lib.lib().p3d_conv_gemm(ctypes.byref(a), _lib.stream_ptr()), 'p3d_conv_gemm', flops, split)
+    native.timed_call(_conv_event(flops, split), 'p3d_conv_gemm', ctypes.byref(a), device=x.device)
     return out
 
 
 def conv_gemm_try(x, w, cout, taps, grid_hw, out, split=False, **kw):
     """conv_gemm that reports P3D_UNSUPPORTED (-1) as False instead of raising: for optional fusions (`rgb=`) whose launch shape
     the library decides on; the caller then takes the unfused sequence."""
-    from . import native
     a = _conv_args(x, w, cout, taps, grid_hw, out, split=split, **kw)
-    ev = None
-    if native.kernel_events is not None:
-        ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
-        ev[0].record()
-    with torch.cuda.device(x.device):
-        st = _lib.lib().p3d_conv_gemm(ctypes.byref(a), _lib.stream_ptr())
-    if st == -1:
-        return False
-    if ev is not None:
-        ev[1].record()
-        flops = 2.0 * x.shape[1] * grid_hw[0] * grid_hw[1] * cout * (len(taps) * x.shape[4] + (a.rgb_cout if a.rgb_w else 0))
-        native.kernel_events.append(('conv_gemm', ev[0], ev[1], flops, flops * (3 if split else 1)))
-    _lib.check(st, 'p3d_conv_gemm')
-    _lib.bump()
-    return True
+    flops = 2.0 * x.shape[1] * grid_hw[0] * grid_hw[1] * cout * (len(taps) * x.shape[4] + (a.rgb_cout if a.rgb_w else 0))
+    return native.timed_call(_conv_event(flops, split), 'p3d_conv_gemm', ctypes.byref(a), device=x.device, unsupported_ok=True)
 
 
 TAPS_3X3 = [(ky - 1, kx - 1, ky * 3 + kx) for ky in range(3) for kx in range(3)]
@@ -305,7 +221,7 @@ def conv_transpose3x3_s2(x, w, cout, out, split=False, acc_scale=1.0 / WEIGHT_SC
         taps = tconv_phase_taps(py, px)
         arr[k] = _conv_args(x, w, cout, taps, ghw, out, out_mode=mode, out_map=(2, py, 2, px), split=split, acc_scale=acc_scale)
         flops += 2.0 * b * ghw[0] * ghw[1] * cout * len(taps) * c
-    _launch(x.device, lambda: _lib.lib().p3d_conv_gemm_phases(arr, 4, _lib.stream_ptr()), 'p3d_conv_gemm_phases', flops, split)
+    native.timed_call(_conv_event(flops, split), 'p3d_conv_gemm_phases', arr, 4, device=x.device)
     return out
 
 
@@ -345,29 +261,18 @@ def fir_act_nhwc(x, f, noise, bias, out_planes, out_hw, pad0=(1, 1), fir_gain=4.
     if noise is not None:
         assert noise.is_contiguous() and noise.dtype == torch.float32 and noise.shape[-2:] == (oh, ow)
     sep = separable_factors(f) if (FIR_VARIANT == 3 and not split_in) else None
-    with torch.cuda.device(x.device):
-        if sep is not None:
-            st = _lib.lib().p3d_fir_act_nhwc_sep(_lib.ptr(x), _lib.DTYPE_CODE[x.dtype], sep[0], sep[1], _lib.ptr(noise), _lib.ptr(bias),
-                                                 _lib.ptr(y), out_planes, b, ih, iw, oh, ow, c, pad0[0], pad0[1], fir_gain, act, alpha,
-                                                 act_gain, clamp, nbs, _lib.stream_ptr())
-        elif split_in:
-            st = _lib.lib().p3d_fir_act_nhwc_split(_lib.ptr(x), _lib.ptr(f), _lib.ptr(noise), _lib.ptr(bias), _lib.ptr(y), out_planes, b,
-                                                   ih, iw, oh, ow, c, pad0[0], pad0[1], fir_gain, act, alpha, act_gain, clamp,
-                                                   nbs, _lib.stream_ptr())
-        else:
-            st = _lib.lib().p3d_fir_act_nhwc(_lib.ptr(x), _lib.DTYPE_CODE[x.dtype], _lib.ptr(f), _lib.ptr(noise), _lib.ptr(bias),
-                                             _lib.ptr(y), out_planes, b, ih, iw, oh, ow, c, pad0[0], pad0[1], fir_gain, act, alpha,
-                                             act_gain, clamp, nbs, _lib.stream_ptr())
-    _lib.check(st, 'p3d_fir_act_nhwc')
-    _lib.bump()
+    tail = (out_planes, b, ih, iw, oh, ow, c, pad0[0], pad0[1], fir_gain, act, alpha, act_gain, clamp, nbs)
+    if sep is not None:
+        _lib.call('p3d_fir_act_nhwc_sep', x, _lib.DTYPE_CODE[x.dtype], sep[0], sep[1], noise, bias, y, *tail, device=x.device)
+    elif split_in:
+        _lib.call('p3d_fir_act_nhwc_split', x, f, noise, bias, y, *tail, device=x.device)
+    else:
+        _lib.call('p3d_fir_act_nhwc', x, _lib.DTYPE_CODE[x.dtype], f, noise, bias, y, *tail, device=x.device)
     return y
 
 
 def upsample2x_nhwc(x, f):
     b, h, w, c = x.shape
     y = torch.empty(b, 2 * h, 2 * w, c, device=x.device, dtype=torch.float32)
-    with torch.cuda.device(x.device):
-        st = _lib.lib().p3d_upsample2x_nhwc(_lib.ptr(x), _lib.ptr(f), _lib.ptr(y), b, h, w, c, _lib.stream_ptr())
-    _lib.check(st, 'p3d_upsample2x_nhwc')
-    _lib.bump()
+    _lib.call('p3d_upsample2x_nhwc', x, f, y, b, h, w, c, device=x.device)
     return y

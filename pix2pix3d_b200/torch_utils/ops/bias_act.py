@@ -90,12 +90,8 @@ def _launch(x, b, xref, yref, dy, grad, dim, act_idx, alpha, gain, clamp):
     if x.numel() == 0:
         return y
     step_b = x.stride(dim) if b is not None else 1
-    with torch.cuda.device(x.device):
-        st = _lib.lib().p3d_bias_act(_lib.ptr(x), _lib.ptr(b), _lib.ptr(xref), _lib.ptr(yref), _lib.ptr(dy), _lib.ptr(y),
-                                     _lib.DTYPE_CODE[x.dtype], grad, act_idx, alpha, gain, clamp, x.numel(),
-                                     0 if b is None else b.numel(), step_b, _lib.stream_ptr())
-    _lib.check(st, 'p3d_bias_act')
-    _lib.bump()
+    _lib.call('p3d_bias_act', x, b, xref, yref, dy, y, _lib.DTYPE_CODE[x.dtype], grad, act_idx, alpha, gain, clamp, x.numel(),
+              0 if b is None else b.numel(), step_b, device=x.device)
     return y
 
 

@@ -137,12 +137,8 @@ def _plugin_filtered_lrelu(x, fu, fd, b, si, up, down, px0, px1, py0, py1, sx, s
     a.s_ofs[0], a.s_ofs[1] = sx, sy
     a.sw_limit = (sw_active + 3) >> 2
     a.sign_mode = 1 if write_signs else (2 if read_signs else 0)
-    with torch.cuda.device(x.device):
-        st = _lib.lib().p3d_filtered_lrelu(ctypes.byref(a), _lib.stream_ptr())
-    if st == -1:                                   # P3D_UNSUPPORTED: the reference's rc = -1
-        return None, None, -1
-    _lib.check(st, 'p3d_filtered_lrelu')
-    _lib.bump()
+    if not _lib.call('p3d_filtered_lrelu', ctypes.byref(a), device=x.device, unsupported_ok=True):
+        return None, None, -1                      # P3D_UNSUPPORTED: the reference's rc = -1
     return y, so, 0
 
 
@@ -162,11 +158,8 @@ def _plugin_filtered_lrelu_act_(x, si, sx, sy, gain, slope, clamp, write_signs):
     xst = (_lib.c_int64 * 4)(x.stride(3), x.stride(2), x.stride(1), x.stride(0))
     ss = (_lib.c_int32 * 2)(s.shape[3] << 2, s.shape[2]) if mode else (_lib.c_int32 * 2)(0, 0)
     so_ = (_lib.c_int32 * 2)(sx, sy)
-    with torch.cuda.device(x.device):
-        st = _lib.lib().p3d_filtered_lrelu_act(_lib.ptr(x), _lib.ptr(s) if mode else None, _lib.DTYPE_CODE[x.dtype], xs, xst, ss, so_,
-                                               gain, slope, clamp, mode, _lib.stream_ptr())
-    _lib.check(st, 'p3d_filtered_lrelu_act')
-    _lib.bump()
+    _lib.call('p3d_filtered_lrelu_act', x, s if mode else None, _lib.DTYPE_CODE[x.dtype], xs, xst, ss, so_, gain, slope, clamp, mode,
+              device=x.device)
     return so
 
 

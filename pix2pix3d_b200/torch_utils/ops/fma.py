@@ -55,11 +55,8 @@ def _addcmul(a, b, c):
         return (0,) * len(pad) + tuple(0 if shape[i] == 1 else e.stride(i) for i in range(len(shape)))
 
     arr = ctypes.c_int64 * 4
-    with torch.cuda.device(a.device):
-        st = _lib.lib().p3d_fma(_lib.ptr(a), _lib.ptr(b), _lib.ptr(c), _lib.ptr(out), _lib.DTYPE_CODE[a.dtype], arr(*shape4),
-                                arr(*strides(a)), arr(*strides(b)), arr(*strides(c)), _lib.stream_ptr())
-    _lib.check(st, 'p3d_fma')
-    _lib.bump()
+    _lib.call('p3d_fma', a, b, c, out, _lib.DTYPE_CODE[a.dtype], arr(*shape4), arr(*strides(a)), arr(*strides(b)), arr(*strides(c)),
+              device=a.device)
     return out
 
 

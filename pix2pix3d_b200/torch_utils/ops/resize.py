@@ -28,11 +28,8 @@ def _launch(x, in_hw, out_hw, antialias, transposed):
     n, c = x.shape[:2]
     dst = in_hw if transposed else out_hw
     y = torch.empty(n, c, dst[0], dst[1], device=x.device, dtype=x.dtype)
-    with torch.cuda.device(x.device):
-        st = _lib.lib().p3d_resize_bilinear(_lib.ptr(x), _lib.ptr(y), _lib.DTYPE_CODE[x.dtype], n * c, in_hw[0], in_hw[1],
-                                            out_hw[0], out_hw[1], int(antialias), int(transposed), _lib.stream_ptr())
-    _lib.check(st, 'p3d_resize_bilinear')
-    _lib.bump()
+    _lib.call('p3d_resize_bilinear', x, y, _lib.DTYPE_CODE[x.dtype], n * c, in_hw[0], in_hw[1], out_hw[0], out_hw[1], int(antialias),
+              int(transposed), device=x.device)
     return y
 
 

@@ -126,11 +126,8 @@ def _launch(x, f2d, upx, upy, downx, downy, px0, px1, py0, py1, flip, gain):
     xst = (_lib.c_int64 * 4)(*x.stride())
     ys = (_lib.c_int32 * 4)(*y.shape)
     yst = (_lib.c_int64 * 4)(*y.stride())
-    with torch.cuda.device(x.device):
-        st = _lib.lib().p3d_upfirdn2d(_lib.ptr(x), _lib.ptr(f2d), _lib.ptr(y), _lib.DTYPE_CODE[x.dtype], xs, xst, ys, yst,
-                                      fw, fh, upx, upy, downx, downy, px0, py0, 1 if flip else 0, gain, _lib.stream_ptr())
-    _lib.check(st, 'p3d_upfirdn2d')
-    _lib.bump()
+    _lib.call('p3d_upfirdn2d', x, f2d, y, _lib.DTYPE_CODE[x.dtype], xs, xst, ys, yst, fw, fh, upx, upy, downx, downy, px0, py0,
+              1 if flip else 0, gain, device=x.device)
     return y
 
 

@@ -37,11 +37,7 @@ class _CrossEntropy2d(torch.autograd.Function):
         assert t.shape == (n, h, w) and (wgt is None or wgt.shape == (c,))
         out = torch.empty(2, device=x.device, dtype=torch.float32)          # loss, sum of weights
         ws = torch.empty(CE_WORKSPACE_DOUBLES, device=x.device, dtype=torch.float64)
-        with torch.cuda.device(x.device):
-            st = _lib.lib().p3d_cross_entropy2d_fwd(_lib.ptr(x), _lib.ptr(t), _lib.ptr(wgt), n, c, h * w, IGNORE_INDEX,
-                                                    _lib.ptr(out[0:1]), _lib.ptr(out[1:2]), _lib.ptr(ws), _lib.stream_ptr())
-        _lib.check(st, 'p3d_cross_entropy2d_fwd')
-        _lib.bump(2)
+        _lib.call('p3d_cross_entropy2d_fwd', x, t, wgt, n, c, h * w, IGNORE_INDEX, out[0:1], out[1:2], ws, device=x.device)
         ctx.save_for_backward(x, t, wgt if wgt is not None else x.new_empty(0), out)
         ctx.has_weight = wgt is not None
         return out[0].clone()
@@ -54,10 +50,6 @@ class _CrossEntropy2d(torch.autograd.Function):
         n, c, h, w = x.shape
         g = dloss.to(torch.float32).reshape(1).contiguous()
         gx = torch.empty_like(x)
-        with torch.cuda.device(x.device):
-            st = _lib.lib().p3d_cross_entropy2d_bwd(_lib.ptr(x), _lib.ptr(t), _lib.ptr(wgt) if ctx.has_weight else None,
-                                                    _lib.ptr(g), _lib.ptr(out[1:2]), n, c, h * w, IGNORE_INDEX, _lib.ptr(gx),
-                                                    _lib.stream_ptr())
-        _lib.check(st, 'p3d_cross_entropy2d_bwd')
-        _lib.bump()
+        _lib.call('p3d_cross_entropy2d_bwd', x, t, wgt if ctx.has_weight else None, g, out[1:2], n, c, h * w, IGNORE_INDEX, gx,
+                  device=x.device)
         return gx, None, None

@@ -62,28 +62,6 @@ def test_transposed_conv_phase_taps_cover_the_3x3_kernel_once():
     assert np.allclose(out, ref)
 
 
-def test_conv_args_struct_matches_the_header_field_order():
-    """The ctypes mirror of p3d_conv_args_t ends with the ABI-5 fields in the header's order (a mismatch would shift every
-    pointer after it)."""
-    import os
-    import re
-    from pix2pix3d_b200 import tcconv
-    hdr = open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'include', 'p3d.h')).read()
-    body = hdr[hdr.index('typedef struct {\n    const void* x;'):hdr.index('} p3d_conv_args_t;')]
-    body = re.sub(r'/\*.*?\*/', '', body, flags=re.S)
-    names = []
-    for decl in body.replace('typedef struct {', '').split(';'):
-        decl = decl.strip()
-        if not decl:
-            continue
-        first, *rest = decl.split(',')
-        names.append(re.sub(r'\[.*', '', first.split()[-1].lstrip('*')))
-        names += [re.sub(r'\[.*', '', r.strip().lstrip('*')) for r in rest]
-    mirror = [n for n, _ in tcconv.ConvArgs._fields_]
-    rename = {'up_filter': 'up_filter'}
-    assert [rename.get(n, n) for n in names] == mirror
-
-
 def test_fma_cpu_path_and_unbroadcast():
     from pix2pix3d_b200.torch_utils.ops import fma
     torch.manual_seed(0)

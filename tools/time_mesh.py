@@ -88,19 +88,16 @@ def main():
     del sigma_np
 
     # marching cubes: the two C entry points, timed with events
-    lib = _lib.lib()
-    ws_bytes = lib.p3d_marching_cubes_workspace_bytes(R, R, R)
+    ws_bytes = _lib.lib().p3d_marching_cubes_workspace_bytes(R, R, R)
     work = torch.empty(ws_bytes, device=dev, dtype=torch.uint8)
     counts = torch.empty(2, device=dev, dtype=torch.int64)
     c_thr = ctypes.c_double(thr)
-    count = lambda: _lib.check(lib.p3d_marching_cubes_count(_lib.ptr(grid), R, R, R, c_thr, _lib.ptr(work), ws_bytes,
-                                                            _lib.ptr(counts), _lib.stream_ptr()), 'count')
+    count = lambda: _lib.call('p3d_marching_cubes_count', grid, R, R, R, c_thr, work, ws_bytes, counts, device=dev)
     count()
     V, F = counts.tolist()
     verts = torch.empty(V, 3, device=dev, dtype=torch.float64)
     faces = torch.empty(F, 3, device=dev, dtype=torch.int64)
-    emit = lambda: _lib.check(lib.p3d_marching_cubes_emit(_lib.ptr(grid), R, R, R, c_thr, _lib.ptr(work), ws_bytes,
-                                                          _lib.ptr(verts), _lib.ptr(faces), _lib.stream_ptr()), 'emit')
+    emit = lambda: _lib.call('p3d_marching_cubes_emit', grid, R, R, R, c_thr, work, ws_bytes, verts, faces, device=dev)
     emit()
     res['vertices'], res['faces'] = V, F
     res['count_ms'] = round(event_ms(count, args.iters), 4)
